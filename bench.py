@@ -2,6 +2,7 @@
 """bench.py -- images/sec of the ViT-B/16 224^2 bf16 forward pass (BASELINE.json `metric`, configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config vit_b16|vit_l16_384|...]
+                    [--dump-outputs DIR]
 
 One "step" is one forward pass over one synthetic batch (256 images per GPU).  N > 1 is launched by torchrun, one
 rank per GPU: the batch is sharded data-parallel (weak scaling: 256 images per GPU), the forward has no
@@ -16,6 +17,10 @@ communication and ends with ONE NCCL all-gather of the logits.  Rank 0 prints ON
 `cpu_baseline` the oracle's torch-CPU restatement of the reference (TensorFlow is not installable here) on a
                bounded sample, on the host cores of the same box.
 `--impl reference` times that CPU restatement as the reference arm.
+
+`--dump-outputs DIR` writes, after the timed steps, what the timed path returned in its last step: `DIR/logits.npy`, float32
+[global batch, classes] (for `--impl reference`, the CPU restatement's logits of its sample).  Weights and images come from
+fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -30,6 +35,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark leaves the tree it runs from untouched (no __pycache__)
 
 CONFIGS = {
     # BASELINE.json configs[1] -- the configuration the metric is quoted on
@@ -161,7 +167,8 @@ def usable_cores():
 
 # --------------------------------------------------------------------------------------------- CPU arm
 def time_cpu_reference(c, budget_s, steps, warmup, log=None):
-    """Restated reference (oracle/ref_torch.py, torch CPU fp32, all host threads) on a bounded sample."""
+    """Restated reference (oracle/ref_torch.py, torch CPU fp32, all host threads) on a bounded sample.  `budget_s` (None: no
+    budget) stops the timed loop early once exceeded; returns (summary, ms per forward, batch, logits of the last forward)."""
     import numpy as np
     import torch
     import oracle
@@ -177,22 +184,25 @@ def time_cpu_reference(c, budget_s, steps, warmup, log=None):
     for _ in range(warmup):
         ref(img)
     ts = []
+    out = None
     for _ in range(steps):
-        t0 = time.perf_counter(); ref(img); ts.append(time.perf_counter() - t0)
-        if time.perf_counter() - t_start > budget_s and len(ts) >= 1:
+        t0 = time.perf_counter(); out = ref(img); ts.append(time.perf_counter() - t0)
+        if budget_s is not None and time.perf_counter() - t_start > budget_s:
             break
     steps = len(ts)
     t = sum(ts) / len(ts)
     return dict(value=b / t, unit="images/s", cores=cores, kind="port",
                 sample=f"{steps} timed forwards of a {b}-image batch after {warmup} warm-up (torch {torch.__version__} CPU fp32 "
-                       f"restatement of vit_tensorflow; TensorFlow not installable in this image)"), t * 1e3, b
+                       f"restatement of vit_tensorflow; TensorFlow not installable in this image)"), t * 1e3, b, out
 
 
 def run_reference(args, c):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    cb, ms, b = time_cpu_reference(c, budget_s=150.0, steps=args.steps, warmup=args.warmup)
+    cb, ms, b, out = time_cpu_reference(c, budget_s=None, steps=args.steps, warmup=args.warmup)
+    if args.dump_outputs:
+        dump_logits(args.dump_outputs, out)
     line = dict(impl="reference", metric=metric_name(args.config), value=cb["value"], unit="images/s", n_gpus=args.gpus, steps=args.steps,
                 warmup=args.warmup, ms_per_step=ms, higher_is_better=True, scaling="weak", vs_baseline=None, dtype="f32",
                 data="synthetic", config=dict(workload=args.config, kind=c["kind"], sample_batch=b,
@@ -258,10 +268,11 @@ def run_ours(args, c):
     barrier()
     ev0.record()
     for _ in range(args.steps):
-        dp.forward_device(img_dev)
+        out_dev = dp.forward_device(img_dev)
     ev1.record()
     barrier()
     ms_total = max_over_ranks(ev0.elapsed_time(ev1))
+    last_logits = out_dev.float().cpu().numpy() if args.dump_outputs else None     # the buffer is reused by the passes below
     # the same K steps again with per-kernel-class CUDA events on the launch stream (roofline numbers); the event
     # records between kernels defeat programmatic dependent launch, so this pass is a little slower than `value`
     model.profile(True)
@@ -347,7 +358,7 @@ def run_ours(args, c):
                           power_w_max=clocks.get("power_w_max"), power_limit_w=clocks.get("power_limit_w"))
         cb = None
         if world == 1 and not args.no_cpu_baseline:
-            cb, _, _ = time_cpu_reference(c, budget_s=20.0, steps=3, warmup=1)
+            cb, _, _, _ = time_cpu_reference(c, budget_s=20.0, steps=3, warmup=1)
         line = dict(metric=metric_name(args.config), value=value, unit="images/s", n_gpus=world, steps=args.steps, warmup=max(args.warmup, 3),
                     ms_per_step=ms_step, higher_is_better=True, scaling="weak", vs_baseline=None,
                     dtype="bf16" if args.precision == "bf16" else "f32", data="synthetic",
@@ -361,9 +372,21 @@ def run_ours(args, c):
                     e2e=e2e, gpu_launches=int(launches_per_step * args.steps), clocks=clocks_out, roofline=roof,
                     cpu_baseline=cb, tflops_end_to_end=value * flops_img / 1e12, e2e_checksum=checksum)
         print(json.dumps(line), flush=True)
+        if args.dump_outputs:
+            dump_logits(args.dump_outputs, last_logits)
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+def dump_logits(directory, logits):
+    """DIR/logits.npy, float32; at most 64 MB (the logits of every configuration here at its default batch are about 1 MB)."""
+    import numpy as np
+    a = np.ascontiguousarray(logits, dtype=np.float32)
+    if a.nbytes > 64 << 20:
+        raise SystemExit(f"--dump-outputs: logits of {a.nbytes >> 20} MB exceed the 64 MB a dump may take")
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "logits.npy"), a)
 
 
 def main():
@@ -377,7 +400,11 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="override the per-GPU batch of the config")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--torch-dp", action="store_true", help="N > 1: torch.distributed for the all-gather instead of the C-ABI's own NCCL path")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's logits to DIR/logits.npy (float32) for output-for-output comparison of builds")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     c = dict(CONFIGS[args.config])
     if args.batch:
         c["batch"] = args.batch

@@ -1,4 +1,6 @@
 """Shared model configurations for the parity tests (small enough for the CPU oracle to finish in seconds)."""
+import json
+
 import numpy as np
 
 import oracle
@@ -74,6 +76,99 @@ README = {
     "t2t_readme": dict(kind="t2t_vit", image_size=224, num_classes=1000, dim=512, depth=5, heads=8, mlp_dim=512,
                        t2t_layers=((7, 4), (3, 2), (3, 2))),
 }
+
+
+# The drop-in classes and the reference classes they stand for: (our class, reference module, reference class).
+REFERENCE_PAIRS = [("ViT", "vit", "ViT"), ("DeepViT", "deepvit", "DeepViT"), ("CaiT", "cait", "CaiT"), ("CrossViT", "cross_vit", "CrossViT"),
+                   ("ParallelViT", "parallel_vit", "ViT"), ("T2TViT", "t2t", "T2TViT"), ("PatchMergerViT", "vit_with_patch_merger", "ViT"),
+                   ("EfficientViT", "efficient", "ViT"), ("PatchMerger", "vit_with_patch_merger", "PatchMerger")]
+CALL_PAIRS = REFERENCE_PAIRS + [("DistillableViT", "distill", "DistillableViT")]
+
+# Constructor kwargs every one of which the reference's constructor rejects: (our class, reference module, reference class, kwargs).
+CTOR_ERROR_CASES = [
+    ("ViT", "vit", "ViT", dict(image_size=30, patch_size=16, num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32)),
+    ("ViT", "vit", "ViT", dict(image_size=32, patch_size=16, num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32, pool="max")),
+    ("ViT", "vit", "ViT", dict(image_size=(32, 40), patch_size=(16, 16), num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32)),
+    ("DeepViT", "deepvit", "DeepViT", dict(image_size=30, patch_size=16, num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32)),
+    ("DeepViT", "deepvit", "DeepViT", dict(image_size=32, patch_size=16, num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32, pool="sum")),
+    ("CaiT", "cait", "CaiT", dict(image_size=30, patch_size=16, num_classes=4, dim=32, depth=1, cls_depth=1, heads=2, mlp_dim=32)),
+    ("CrossViT", "cross_vit", "CrossViT", dict(image_size=30, num_classes=4, sm_dim=32, lg_dim=32)),
+    ("ParallelViT", "parallel_vit", "ViT", dict(image_size=30, patch_size=16, num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32)),
+    ("T2TViT", "t2t", "T2TViT", dict(image_size=32, num_classes=4, dim=32)),
+    ("T2TViT", "t2t", "T2TViT", dict(image_size=32, num_classes=4, dim=32, depth=1, heads=2, mlp_dim=32, pool="max")),
+    ("PatchMergerViT", "vit_with_patch_merger", "ViT", dict(image_size=30, patch_size=16, num_classes=4, dim=32, depth=2, heads=2, mlp_dim=32)),
+    ("EfficientViT", "efficient", "ViT", dict(image_size=30, patch_size=16, num_classes=4, dim=32, transformer=None)),
+    ("EfficientViT", "efficient", "ViT", dict(image_size=32, patch_size=16, num_classes=4, dim=32, transformer=None, pool="max")),
+]
+
+NO_DEFAULT = "<no default>"       # how tests/golden/reference_boundary.json spells a parameter without a default
+
+
+def error_case_id(ours, kw):
+    """The key of a CTOR_ERROR_CASES entry in tests/golden/reference_boundary.json."""
+    return f"{ours} {json.dumps(kw, sort_keys=True)}"
+
+
+RANDOM_KINDS = ["vit", "deepvit", "cait", "crossvit", "parallel_vit", "patch_merger_vit", "t2t_vit"]
+RANDOM_SEEDS = 40
+
+
+def random_case(kind, rng):
+    """A random small constructor-kwargs set of `kind` (every shape-changing argument drawn, incl. the branches the hand-picked
+    cases might miss: rectangular images, heads == 1 with dim_head == dim (no out-projection, vit.py:53), equal CrossViT widths
+    (no ProjectInOut Dense, cross_vit.py:124), PatchMerger after the first / last layer, T2T kernel / stride combinations)."""
+    heads = int(rng.choice([1, 2, 3]))
+    dim_head = int(rng.choice([4, 8]))
+    dim = heads * dim_head if (heads == 1 and rng.random() < 0.5) else int(rng.choice([8, 12, 20]))
+    base = dict(num_classes=int(rng.integers(2, 7)), dim=dim, depth=int(rng.integers(1, 4)), heads=heads, mlp_dim=int(rng.choice([8, 24])),
+                dim_head=dim_head)
+    if kind in ("vit", "parallel_vit", "patch_merger_vit"):
+        ph, pw = int(rng.choice([2, 4])), int(rng.choice([2, 4]))
+        case = dict(kind=kind, image_size=(ph * int(rng.integers(1, 4)), pw * int(rng.integers(1, 4))), patch_size=(ph, pw), **base)
+        if kind != "patch_merger_vit":
+            case["pool"] = str(rng.choice(["cls", "mean"]))
+        if kind == "parallel_vit":
+            case["num_parallel_branches"] = int(rng.integers(1, 4))
+        if kind == "patch_merger_vit":
+            case["depth"] = int(rng.integers(2, 5))
+            case["patch_merge_layer"] = int(rng.integers(1, case["depth"] + 1)) if rng.random() < 0.7 else None
+            case["patch_merge_num_tokens"] = int(rng.integers(1, 5))
+        return case
+    if kind in ("deepvit", "cait"):
+        p = int(rng.choice([2, 4]))
+        case = dict(kind=kind, image_size=p * int(rng.integers(1, 4)), patch_size=p, **base)
+        if kind == "deepvit":
+            case["pool"] = str(rng.choice(["cls", "mean"]))
+        else:
+            case["cls_depth"] = int(rng.integers(1, 3))
+        return case
+    if kind == "t2t_vit":
+        layers = tuple((int(rng.choice([3, 5])), int(rng.choice([1, 2]))) for _ in range(int(rng.integers(1, 3))))
+        return dict(kind=kind, image_size=int(rng.choice([6, 8, 9])), t2t_layers=layers, pool=str(rng.choice(["cls", "mean"])), **base)
+    if kind == "crossvit":
+        sm_dim = int(rng.choice([8, 12]))
+        lg_dim = sm_dim if rng.random() < 0.4 else int(rng.choice([16, 20]))
+        return dict(kind=kind, image_size=16, num_classes=int(rng.integers(2, 6)), sm_dim=sm_dim, lg_dim=lg_dim, sm_patch_size=int(rng.choice([4, 8])),
+                    lg_patch_size=int(rng.choice([8, 16])), sm_enc_depth=int(rng.integers(1, 3)), lg_enc_depth=int(rng.integers(1, 3)),
+                    sm_enc_heads=int(rng.choice([1, 2])), lg_enc_heads=int(rng.choice([1, 2])), sm_enc_mlp_dim=8, lg_enc_mlp_dim=12,
+                    sm_enc_dim_head=4, lg_enc_dim_head=8, cross_attn_depth=int(rng.integers(1, 3)), cross_attn_heads=int(rng.choice([1, 3])),
+                    cross_attn_dim_head=4, depth=int(rng.integers(1, 3)))
+    raise ValueError(kind)
+
+
+def random_configuration(kind, seed):
+    """(case, cfg) of random configuration `seed` of `kind`.  T2T draws the reference cannot run are redrawn: the reference sizes
+    pos_embedding with a conv formula (t2t.py:14-15,66,76) but tokenises with SAME padding (:43); when the formula comes out short
+    its own call fails at :102 -- not a configuration anyone can run."""
+    rng = np.random.default_rng(1000 * seed + len(kind))
+    while True:
+        case = random_case(kind, rng)
+        cfg = oracle.make_config(kind, **{k: v for k, v in case.items() if k != "kind"})
+        if kind != "t2t_vit":
+            return case, cfg
+        gh, gw = oracle.t2t_token_grid(cfg)[-1]
+        if cfg["num_patches"] >= gh * gw:
+            return case, cfg
 
 
 def cfg_of(name):

@@ -6,11 +6,13 @@ marshalling, attribute surface -- runs here), and oracle/tf_shim.py lets the ref
 
 * host classes over the double: every stage entry goes through the real marshalling code and reproduces the oracle; what comes
   back answers `.numpy()` like the eager tensors the reference returns; `patch_embedding.layers[1].weights` exists;
-* LIVE (reference checkout present): the UNMODIFIED `simmim.SimMIM`, `mae.MAE`, `mpp.MPP` and `distill.DistillWrapper` are
-  constructed around (a) the reference's own ViT and (b) our ViT carrying the same weights, with the same random stream: the
-  losses agree, i.e. every attribute and call those wrappers make on their encoder (mae.py:32-38,49-69, simmim.py:74-80,88-125,
-  mpp.py:149,200-212, distill.py:96-117) works on the drop-in and means the same thing.
+* the reference's wrappers: the UNMODIFIED `simmim.SimMIM`, `mae.MAE`, `mpp.MPP` and `distill.DistillWrapper`, constructed
+  around (a) the reference's own ViT and (b) our ViT carrying the same weights, with the same random stream, give the same
+  loss, i.e. every attribute and call those wrappers make on their encoder (mae.py:32-38,49-69, simmim.py:74-80,88-125,
+  mpp.py:149,200-212, distill.py:96-117) works on the drop-in and means the same thing.  tests/golden/make_wrapper_interactions.py
+  checks that where the reference checkout exists and records run (a); the tests below replay it on the drop-in.
 """
+import json
 import os
 
 import numpy as np
@@ -18,10 +20,7 @@ import pytest
 
 import oracle
 import fake_engine
-from oracle import ref_bind, spec_numpy, tf_shim
-
-REF_DIR = os.environ.get("VB_REFERENCE_DIR", "/root/reference/vit_tensorflow")    # the reference checkout (absent on the GPU box)
-live = pytest.mark.skipif(not os.path.isdir(REF_DIR), reason="reference checkout not present (GPU box)")
+from oracle import spec_numpy
 
 KW = dict(image_size=64, patch_size=16, num_classes=10, dim=64, depth=2, heads=4, mlp_dim=128, dim_head=16)
 CFG = oracle.make_config("vit", **KW)
@@ -82,82 +81,104 @@ def test_distillable_vit_over_the_double():
         assert m.dim == 64 and m.num_classes == 10 and hasattr(logits, "numpy")       # distill.py:96-97
 
 
-# ------------------------------------------------------------------------------------------ live: the reference's wrappers
-def _encoders():
-    """(label, factory) pairs: the reference's ViT with W loaded, and ours with W loaded.  Call inside the installed() blocks."""
-    return [("reference", lambda: ref_bind.build_model("vit", KW, W, IMG)), ("ours", _ours)]
+# ------------------------------------------------------------------------------------------ the reference's wrappers, replayed
+# What the reference's unmodified wrappers did to the reference's own ViT -- every attribute read and every call, with its
+# arguments and result -- is stored in tests/golden/wrapper_interactions__refshim.npz.  tests/golden/make_wrapper_interactions.py
+# recorded it and, running each wrapper around our ViT as well, checked that the wrapper makes the same interactions there and
+# ends with the same loss.  Here every interaction is replayed on our encoder and must give back what the reference's gave: the
+# wrapper's computation is a function of those answers and its own seeded random stream, so equal answers are an equal loss.
+REPLAY_TOL = 1e-5
 
 
-def _run_wrapper(build, call):
-    out = {}
-    for label, factory in _encoders():
-        with fake_engine.installed() as fake, tf_shim.installed(REF_DIR):
-            enc = factory()
-            tf_shim.set_seed(77)                      # same random stream for the wrapper's own variables and masks in both runs
-            wrapper = build(enc)
-            tf_shim.set_seed(78)
-            out[label] = (float(call(wrapper)), [c[0] for c in fake.calls])
-    return out
+def img_patches(img):
+    """The images cut into 16 x 16 patches, 'b (h p1) (w p2) c -> b (h w) (p1 p2 c)' (one of the stored interactions' inputs)."""
+    from einops import rearrange
+    return rearrange(img, "b (h p1) (w p2) c -> b (h w) (p1 p2 c)", p1=16, p2=16)
 
 
-@live
-def test_live_simmim_over_the_dropin_encoder():
-    def build(enc):
-        import simmim
-        return simmim.SimMIM(image_size=64, encoder=enc, masking_ratio=0.5)
-    r = _run_wrapper(build, lambda w: w(IMG, training=False))
-    assert np.isfinite(r["ours"][0]) and abs(r["ours"][0] - r["reference"][0]) < 1e-6
-    assert r["ours"][1] == ["vb_create", "vb_finalize", "vb_to_patch", "vb_patch_to_emb", "vb_forward_tokens"] and r["reference"][1] == []
+@pytest.fixture(scope="module")
+def interactions():
+    z = np.load(os.path.join(os.path.dirname(__file__), "golden", "wrapper_interactions__refshim.npz"))
+    return json.loads(str(z["meta"]))["wrappers"], {k: z[k] for k in z.files if k != "meta"}
 
 
-@live
-def test_live_mae_over_the_dropin_encoder():
-    def build(enc):
-        import mae
-        return mae.MAE(image_size=64, encoder=enc, decoder_dim=32, masking_ratio=0.75, decoder_depth=1, decoder_heads=2, decoder_dim_head=16)
-    r = _run_wrapper(build, lambda w: w(IMG, training=False))
-    assert np.isfinite(r["ours"][0]) and abs(r["ours"][0] - r["reference"][0]) < 1e-6
-    assert r["ours"][1][-1] == "vb_forward_tokens"                                  # the encoder saw only the unmasked quarter (mae.py:63-69)
+def _replay(recorded, name, encoder):
+    """Replays wrapper `name`'s recorded interactions on `encoder`; returns the number replayed."""
+    wrappers, arrays = recorded
+    known = {"img": IMG, "img_patches": img_patches(IMG), **{f"w:{k}": v for k, v in W.items()}}
+
+    def arg(d):
+        if "tuple" in d:
+            return tuple(arg(e) for e in d["tuple"])
+        if "py" in d:
+            return tuple(d["py"]) if isinstance(d["py"], list) else d["py"]
+        if "array" in d:
+            return arrays[d["array"]]
+        a = np.asarray(known[d["ref"]], dtype=np.float32)
+        if "rows" in d:                               # each row: a row of the reference (>= 0) or one of the stored other rows
+            base, other = a.reshape(-1, a.shape[-1]), arrays[d["other"]]
+            a = np.stack([base[i] if i >= 0 else other[-1 - i] for i in arrays[d["rows"]]]).reshape(a.shape)
+        return a
+
+    def check(got, d, where):
+        if "tuple" in d:
+            assert isinstance(got, tuple) and len(got) == len(d["tuple"]), where
+            for g, e in zip(got, d["tuple"]):
+                check(g, e, where)
+        elif "py" in d:
+            assert (list(got) if isinstance(got, tuple) else got) == d["py"], (where, got, d["py"])
+        else:
+            want = arg(d)
+            assert np.shape(got) == want.shape, where
+            np.testing.assert_allclose(np.asarray(got, np.float32), want, rtol=0, atol=REPLAY_TOL, err_msg=str(where))
+
+    events = wrappers[name]["events"]
+    for i, e in enumerate(events):
+        target = encoder
+        for kind, step in e["path"]:
+            target = getattr(target, step) if kind == "attr" else target[step]
+        if e["op"] == "get":
+            check(target, e["value"], (name, i, e["path"]))
+            continue
+        got = target(*[arg(a) for a in e["args"]], **{k: arg(v) for k, v in e["kwargs"].items()})
+        check(got, e["result"], (name, i, e["path"]))
+        if isinstance(got, np.ndarray):
+            known[f"result:{i}"] = got                # later arguments built from this answer use ours, as the wrapper would
+    return len(events)
 
 
-@live
-def test_live_mpp_over_the_dropin_encoder():
+def _replay_on_ours(interactions, name, cls_name="ViT"):
+    with fake_engine.installed() as fake:
+        n = _replay(interactions, name, _ours(cls_name))
+        calls = [c[0] for c in fake.calls]
+    assert n > 0 and calls == interactions[0][name]["engine_calls"]
+    return calls
+
+
+def test_live_simmim_over_the_dropin_encoder(interactions):
+    """simmim.SimMIM around the drop-in (simmim.py:74-80,88-125): pos_embedding, patch_embedding.layers[:2] and their weights,
+    to_patch / patch_to_emb / transformer on the wrapper's own inputs."""
+    calls = _replay_on_ours(interactions, "simmim")
+    assert calls == ["vb_create", "vb_finalize", "vb_to_patch", "vb_patch_to_emb", "vb_forward_tokens"]
+
+
+def test_live_mae_over_the_dropin_encoder(interactions):
+    calls = _replay_on_ours(interactions, "mae")
+    assert calls[-1] == "vb_forward_tokens"                                         # the encoder saw only the unmasked quarter (mae.py:63-69)
+
+
+def test_live_mpp_over_the_dropin_encoder(interactions):
     """mpp.py:200-212: Dense of `patch_embedding.layers[-1]` on masked patches, cls token, `pos_embedding[:, :(n + 1)]`, `dropout`,
-    `transformer`.  MPP's own loss is degenerate on these inputs (it is 0 on both encoders), so the probe compares the logits MPP
-    computes from the encoder's output instead."""
-    seen = {}
-
-    def build(enc):
-        import mpp
-        w = mpp.MPP(image_size=64, transformer=enc, patch_size=16, mask_prob=0.15, random_patch_prob=0.30, replace_prob=0.50)
-        w.loss = lambda logits, img, mask: seen.setdefault(len(seen), np.asarray(logits)).mean()    # instrumentation on the INSTANCE
-        return w
-    r = _run_wrapper(build, lambda w: w(IMG, training=False))
-    assert seen[0].shape == (3, 16, 512) and np.abs(seen[0] - seen[1]).max() < 1e-5
-    assert r["ours"][1] == ["vb_create", "vb_finalize", "vb_patch_to_emb", "vb_forward_tokens"]
+    `transformer`."""
+    calls = _replay_on_ours(interactions, "mpp")
+    assert calls == ["vb_create", "vb_finalize", "vb_patch_to_emb", "vb_forward_tokens"]
 
 
-@live
-def test_live_distill_wrapper_over_the_dropin_student(hard=False):
+def test_live_distill_wrapper_over_the_dropin_student(interactions):
     """distill.py:87-136: `student.dim`, `student.num_classes`, `student(img, distill_token=Variable, training=...)` ->
-    (logits, distill_tokens); the teacher is any callable model.  (soft distillation only: the reference's hard branch feeds
-    integer labels to categorical_crossentropy, distill.py:131-132, which fails on any encoder.)"""
-    out = {}
-    labels = np.eye(10, dtype=np.float32)[[1, 4, 7]]
-    for label in ("reference", "ours"):
-        with fake_engine.installed(), tf_shim.installed(REF_DIR):
-            import distill
-            teacher = ref_bind.build_model("vit", KW, oracle.init_weights(CFG, 9), IMG)
-            student = (ref_bind.build_model("vit", KW, W, IMG, cls=distill.DistillableViT) if label == "reference"
-                       else _ours("DistillableViT"))
-            if label == "ours":
-                # distill.py:91 asserts isinstance(student, (DistillableViT, ...)) against the names in ITS module: the reference-side
-                # binding of the drop-in is therefore `distill.DistillableViT = vit_tensorflow_b200.DistillableViT` (INTEGRATION.md 7)
-                distill.DistillableViT = type(student)
-            tf_shim.set_seed(5)
-            wrapper = distill.DistillWrapper(teacher=teacher, student=student, temperature=3, alpha=0.5, hard=hard)
-            out[label] = np.asarray(wrapper([IMG, labels], training=False), dtype=np.float64)
-    assert np.isfinite(out["ours"]).all() and np.abs(out["ours"] - out["reference"]).max() < 1e-5
+    (logits, distill_tokens).  (soft distillation only: the reference's hard branch feeds integer labels to
+    categorical_crossentropy, distill.py:131-132, which fails on any encoder.)"""
+    _replay_on_ours(interactions, "distill", "DistillableViT")
 
 
 # ------------------------------------------------------------------------------------------ every host class over the double
